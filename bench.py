@@ -6,6 +6,8 @@ obs + reward, SURVEY.md 8d).
   python bench.py --gpus N --steps K --warmup W            this repo's CUDA engine (one process per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  the CPU restatement of the reference loop (oracle/ref_env.py
                                                            over oracle/fe_oracle.c) on all host cores; rank 0 only
+  python bench.py ... --dump-outputs DIR                   also write what the last timed step returned (DIR/<name>.npy):
+                                                           the inputs are seeded, so two builds can be compared output for output
 
 Prints ONE JSON line (see the contract in the task statement / DESIGN.md "Measurement").
 """
@@ -76,6 +78,21 @@ class ClockSampler(threading.Thread):
         self.join(timeout=2)
         return {"sm_mhz": statistics.median(self.samples) if self.samples else None, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(self.samples)}
+
+
+def dump_outputs(tensors, out_dir, max_bytes=64 << 20):
+    """<out_dir>/<name>.npy of every tensor: floats as float32, the integer and boolean ones as float64 (exact for int32).  Above
+    `max_bytes` in all, every array keeps the same fixed, seeded fraction of its rows."""
+    import numpy as np
+
+    arrays = {n: t.cpu().numpy() for n, t in tensors.items()}
+    arrays = {n: a.astype(np.float32 if a.dtype.kind == "f" else np.float64) for n, a in arrays.items()}
+    frac = min(1.0, (max_bytes - 128 * len(arrays)) / sum(a.nbytes for a in arrays.values()))  # 128: an .npy header
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in arrays.items():
+        if frac < 1.0:
+            a = a[np.sort(np.random.RandomState(0).choice(len(a), int(len(a) * frac), replace=False))]
+        np.save(os.path.join(out_dir, n + ".npy"), a)
 
 
 def build_id():
@@ -284,7 +301,7 @@ def run_ours(args):
     for k in range(K):
         flush.fill_(float(k))  # evict L2 between timed iterations (not timed)
         ev[k][0].record()
-        env.step(acts[W + k])
+        last = env.step(acts[W + k])
         ev[k][1].record()
     barrier()
     clocks = sampler.stop()
@@ -404,6 +421,9 @@ def run_ours(args):
             v, n = cpu_env_rate(args.cpu_seconds)
             out["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": 1, "kind": "port",
                                    "sample": "%d env.step() of one CPU oracle env (oracle/ref_env.py over oracle/fe_oracle.c) in %.0f s" % (n, args.cpu_seconds)}
+        if args.dump_outputs:  # leg 1's env is not stepped after its timed window: its buffers still hold that window's last step
+            od, rew, done, info = last
+            dump_outputs(dict(od, reward=rew, done=done, info=info), args.dump_outputs)
         print(json.dumps(out))
     if dist is not None:
         dist.barrier()
@@ -426,7 +446,12 @@ def main():
     ap.add_argument("--reward", default="sparse", choices=["sparse", "dense"], help="dense = FurnitureSawyerDenseRewardEnv (IKEASawyerDense-v0), one GPU, not the bench line")
     ap.add_argument("--ref-slice", type=float, default=1.0, help="--impl reference: seconds every worker runs free per bench step")
     ap.add_argument("--actions", default="random", choices=["random", "settled"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the observations, rewards, dones and infos of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

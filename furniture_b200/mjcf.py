@@ -131,14 +131,10 @@ def _floats(s, n=None, default=None):
 # scene composition (reference composer restated)
 # --------------------------------------------------------------------------------------
 
-REFERENCE_ASSETS = "/root/reference/furniture/env/models/assets"
-
-
 def default_assets_root():
-    for cand in (os.environ.get("FURNITURE_ASSETS"), REFERENCE_ASSETS):
-        if cand and os.path.isdir(cand):
-            return cand
-    return None
+    """the reference's MJCF asset tree (furniture/env/models/assets) named by FURNITURE_ASSETS, or None"""
+    cand = os.environ.get("FURNITURE_ASSETS")
+    return cand if cand and os.path.isdir(cand) else None
 
 
 def furniture_names(assets_root):

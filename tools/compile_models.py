@@ -1,7 +1,7 @@
 """Compile the composed MJCF scenes into flat tables (furniture_b200/compiled/*.npz).
 
-Runs where the reference asset tree is reachable (build container).  The GPU box has no /root/reference, so the
-package falls back to these tables (mjcf.load_scene).  Only derived numeric tables are stored, no reference source."""
+Needs the reference's MJCF asset tree, named by FURNITURE_ASSETS.  Without it the package loads these tables
+(mjcf.load_scene).  Only derived numeric tables are stored, no reference source."""
 import os
 import sys
 
